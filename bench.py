@@ -8,6 +8,13 @@ A "step" = one search() of all nq queries over the whole database.
   python bench.py --impl reference --gpus 1 --steps K ...   # reference CPU IndexFlatL2 (oracle/_ref)
   torchrun --nproc-per-node N bench.py --gpus N ...         # database sharded over N GPUs
                                                             # (IndexShards semantics, NCCL all-gather merge)
+  python bench.py ... --dump-outputs DIR                    # also write the last timed step's results to DIR
+
+--steps sets the number of timed steps of every timed loop.  The inputs are seeded: with the same arguments
+(and BENCH_* environment) every run searches the same data, so the files of --dump-outputs from two builds can
+be compared array for array: DIR/flat_D.npy (float32 [nq, k] distances) and DIR/flat_I.npy (float64 [nq, k]
+ids), and at one GPU ivfpq_{D,I}.npy and ivfpq_synthetic_{D,I}.npy of the IVFPQ workloads (36 MB in all at
+the default sizes; larger results are cut to a fixed set of query rows, see dump_outputs).
 
 One JSON line on stdout (rank 0).  `value` = QPS with inputs resident in HBM; `e2e` = QPS through
 the public API with host (pinned) buffers, H2D/D2H inside the timed region; `roofline` = algorithmic
@@ -45,6 +52,26 @@ UNIT = "queries/s"
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+DUMP_BYTES_PER_WORKLOAD = 20 << 20  # three workloads stay under 64 MB
+
+
+def dump_outputs(dirname, name, D, I):
+    """one timed step's search result as DIR/<name>_D.npy (float32) and DIR/<name>_I.npy (float64: ids < 2^53 are
+    exact).  A result larger than DUMP_BYTES_PER_WORKLOAD is cut to evenly spaced query rows, whose indices go to
+    DIR/<name>_rows.npy."""
+    if not dirname:
+        return
+    os.makedirs(dirname, exist_ok=True)
+    D, I = D.cpu().numpy(), I.cpu().numpy()
+    row_bytes = D.shape[1] * 12
+    if D.shape[0] * row_bytes > DUMP_BYTES_PER_WORKLOAD:
+        rows = np.linspace(0, D.shape[0] - 1, DUMP_BYTES_PER_WORKLOAD // row_bytes).astype(np.int64)
+        D, I = D[rows], I[rows]
+        np.save(os.path.join(dirname, name + "_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(dirname, name + "_D.npy"), np.asarray(D, dtype=np.float32))
+    np.save(os.path.join(dirname, name + "_I.npy"), np.asarray(I, dtype=np.float64))
 
 
 def peaks():
@@ -406,7 +433,7 @@ def _recalls(I, gt):
     return out
 
 
-def ivfpq_workload(torch, fb, res, device, name, N, d, nlist, M, nprobe, nq, k, steps, warmup, data, n_gt, cpu_queries):
+def ivfpq_workload(torch, fb, res, device, name, N, d, nlist, M, nprobe, nq, k, steps, warmup, data, n_gt, cpu_queries, dump_dir=None):
     """Build a GpuIndexIVFPQ, time search (device-resident and e2e), clone it to the reference CPU
     IndexIVFPQ (same centroids / PQ / list bytes), time that on the host cores, report recall for both.
     data = ("uniform", None) -> seeded uniform chunks generated on the device;
@@ -494,6 +521,7 @@ def ivfpq_workload(torch, fb, res, device, name, N, d, nlist, M, nprobe, nq, k, 
     for _ in range(steps):
         index.search(xq_pin.numpy(), k, D=D_pin.numpy(), I=I_pin.numpy())
     e2e_ms = (time.time() - t0) * 1e3 / steps
+    dump_outputs(dump_dir, name, D, I)
 
     gpu_I = I[:n_gt].cpu().numpy()
     gpu_D = D[:n_gt].cpu().numpy()
@@ -602,8 +630,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-ivfpq", action="store_true", help="skip the IVFPQ workloads (configs[3] + SyntheticDataset)")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last timed step's results to DIR as .npy (rank 0)")
     args = ap.parse_args()
-    steps, warmup = max(1, args.steps), max(0, args.warmup)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    steps, warmup = args.steps, max(0, args.warmup)
 
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -728,6 +760,8 @@ def main():
         step_e2e()
     barrier()
     e2e_ms = (time.time() - t0) * 1e3 / steps
+    if rank == 0:
+        dump_outputs(args.dump_outputs, "flat", D, I)
 
     if dist is not None:
         t = torch.tensor([ms, e2e_ms], dtype=torch.float64, device=device)
@@ -806,15 +840,16 @@ def main():
             wl = {}
             try:
                 n_pq = int(os.environ.get("BENCH_IVFPQ_N", 100_000_000))
-                wl["ivfpq"] = ivfpq_workload(torch, fb, res, device, "ivfpq", n_pq, 128, 4096, 32, 32, NQ, K, min(steps, 10), warmup,
-                                             ("uniform", None), n_gt=1000, cpu_queries=1000)
+                wl["ivfpq"] = ivfpq_workload(torch, fb, res, device, "ivfpq", n_pq, 128, 4096, 32, 32, NQ, K, steps, warmup,
+                                             ("uniform", None), n_gt=1000, cpu_queries=1000, dump_dir=args.dump_outputs)
             except Exception as e:
                 wl["ivfpq"] = {"error": str(e)[:300]}
             try:
                 n_syn = int(os.environ.get("BENCH_SYNTH_N", 2_000_000))
                 xt, xbs, xqs = synthetic_dataset(128, 200_000, n_syn, NQ)
-                wl["ivfpq_synthetic"] = ivfpq_workload(torch, fb, res, device, "ivfpq_synthetic", n_syn, 128, 1024, 32, 32, NQ, K, min(steps, 10), warmup,
-                                                       ("arrays", (xt, xbs, xqs)), n_gt=1000, cpu_queries=1000)
+                wl["ivfpq_synthetic"] = ivfpq_workload(torch, fb, res, device, "ivfpq_synthetic", n_syn, 128, 1024, 32, 32, NQ, K, steps, warmup,
+                                                       ("arrays", (xt, xbs, xqs)), n_gt=1000, cpu_queries=1000,
+                                                       dump_dir=args.dump_outputs)
             except Exception as e:
                 wl["ivfpq_synthetic"] = {"error": str(e)[:300]}
             out["workloads"] = wl

@@ -16,7 +16,7 @@ class FaissError(RuntimeError):
 
 if not os.path.exists(LIB_PATH):
     raise ImportError(
-        "faiss_b200: %s is missing. Build it with `python -m faiss_b200.build` (nvcc, sm_100a). "
+        "faiss_b200: %s is missing. Build it with `python faiss_b200/build.py` (nvcc, sm_100a). "
         "There is no CPU fallback." % LIB_PATH
     )
 

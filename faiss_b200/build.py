@@ -1,6 +1,6 @@
 """Build libfaiss_b200.so in-tree with nvcc for sm_100a (no JIT cache, no torch extension).
 
-Usage: python -m faiss_b200.build [-j N] [--force]
+Usage: python faiss_b200/build.py [-j N] [--force]   (a script: importing the package needs the library it builds)
 Objects go to faiss_b200/csrc/_obj/, the library to faiss_b200/libfaiss_b200.so.
 """
 import os

@@ -32,19 +32,22 @@ def pytest_collection_modifyitems(config, items):
 
 
 @pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference CPU library (oracle/_ref); skipped where it was never built."""
-    from oracle import ref as r
-
-    if not r.available():
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    return r
-
-
-@pytest.fixture(scope="session")
 def golden():
     path = os.path.join(ROOT, "tests", "golden", "golden.npz")
     return np.load(path)
+
+
+@pytest.fixture(scope="session")
+def ref_outputs():
+    """What the unmodified reference CPU library answered for the inputs of the tests that compare with it
+    (tests/golden/make_reference_outputs.py)."""
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_outputs.npz"))
+
+
+@pytest.fixture(scope="session")
+def ref_outputs_fullsize():
+    """The same for the BASELINE-size configs of tests/test_fullsize_gpu.py (64 sampled queries each)."""
+    return np.load(os.path.join(ROOT, "tests", "golden", "reference_outputs_fullsize.npz"))
 
 
 @pytest.fixture(scope="session")

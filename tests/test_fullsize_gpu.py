@@ -136,7 +136,9 @@ def test_ivfpq_100m_properties(res):
 
 
 # ------------------------------------------------------------------------------------------------
-# BASELINE-size configs against the reference itself (oracle/_ref) on sampled queries.
+# BASELINE-size configs against the reference itself on sampled queries: the answers of the reference CPU library
+# (oracle/_ref) for exactly these inputs and index contents are stored in tests/golden/reference_outputs_fullsize.npz
+# by tests/golden/make_reference_outputs.py, which builds them with the helpers below.
 # Model: faiss/gpu/test/TestUtils.cpp:158-226 (compareLists), TestGpuIndexFlat.cpp, TestGpuIndexIVFFlat.cpp,
 # TestGpuIndexIVFPQ.cpp -- the GPU index and the CPU index hold the SAME data; 64 sampled queries.
 # ------------------------------------------------------------------------------------------------
@@ -148,7 +150,57 @@ def _sample_queries(torch, nq, d, seed, n=64):
     return xq, pick
 
 
-def test_flat_l2_10m_vs_reference(res, ref):
+def flat_10m_inputs(torch):
+    """configs[1]: xb [10M, 128], xq [10k, 128] and the indices of the 64 sampled queries"""
+    N, d, nq = 10_000_000, 128, 10_000
+    xb = _rows(torch, N, d, 1234)
+    xq, pick = _sample_queries(torch, nq, d, 1235)
+    return xb, xq, pick
+
+
+def ivfflat_10m_index(torch, fb, res):
+    """configs[2]: GpuIndexIVFFlat N=10M nlist=4096 nprobe=64.  The coarse centroids are seeded uniform rows (the
+    random-sample start of k-means) rather than a device k-means result: float atomics make the latter vary in the
+    last bits from run to run, and the stored reference answers are only valid for one exact index content."""
+    N, d, nlist, nprobe = 10_000_000, 128, 4096, 64
+    idx = fb.GpuIndexIVFFlat(res, d, nlist, fb.METRIC_L2)
+    idx.setCoarseCentroids(_rows(torch, nlist, d, 4321).cpu().numpy())
+    idx.setIsTrained(True)
+    idx.reserveMemory(N + N // 8)
+    for c0 in range(0, N, 1_000_000):
+        idx.add(_rows(torch, 1_000_000, d, 1234 + c0 // 1_000_000))
+    idx.nprobe = nprobe
+    return idx
+
+
+def sampled_pq_codebooks(torch, cent, M):
+    """PQ codebooks [M, 256, d/M] cut from the residuals of 256 seeded uniform rows to their nearest coarse centroid (the
+    random-sample start of PQ training): reproducible for the reason given in ivfflat_10m_index"""
+    x = _rows(torch, 256, cent.shape[1], 4322).double()
+    c = cent.double()
+    a = ((x * x).sum(1, keepdim=True) - 2 * x @ c.T + (c * c).sum(1)).argmin(dim=1)
+    r = (x - c[a]).float()
+    return r.reshape(256, M, -1).permute(1, 0, 2).contiguous().cpu().numpy()
+
+
+def ivfpq_100m_index(torch, fb, res):
+    """configs[3]: GpuIndexIVFPQ N=100M nlist=4096 M=32 nprobe=32 over seeded uniform coarse centroids (see
+    ivfflat_10m_index) and sampled_pq_codebooks"""
+    N, d, nlist, M, nprobe = 100_000_000, 128, 4096, 32, 32
+    idx = fb.GpuIndexIVFPQ(res, d, nlist, M, 8, fb.METRIC_L2)
+    cent = _rows(torch, nlist, d, 4321)
+    idx.setCoarseCentroids(cent.cpu().numpy())
+    idx.setPQCentroids(sampled_pq_codebooks(torch, cent, M))
+    idx.setIsTrained(True)
+    idx.reserveMemory(N + N // 8)
+    CH = 2_000_000
+    for c0 in range(0, N, CH):
+        idx.add(_rows(torch, CH, d, 1234 + c0 // CH, chunk=CH))
+    idx.nprobe = nprobe
+    return idx
+
+
+def test_flat_l2_10m_vs_reference(res, ref_outputs_fullsize):
     """configs[1] vs faiss::knn_L2sqr over all 10M rows: uniform floats -> compareLists semantics with distances
     <= 1e-4 relative; integer-valued rows -> distances bit-exact and ids exact up to the tie group at rank k."""
     import torch
@@ -156,16 +208,13 @@ def test_flat_l2_10m_vs_reference(res, ref):
     import faiss_b200 as fb
     from oracle import oracle_np as o
 
-    N, d, nq, k = 10_000_000, 128, 10_000, 100
-    xb = _rows(torch, N, d, 1234)
-    xq, pick = _sample_queries(torch, nq, d, 1235)
+    d, k = 128, 100
+    xb, xq, pick = flat_10m_inputs(torch)
     idx = fb.GpuIndexFlatL2(res, d)
     idx.add(xb)
     D, I = idx.search(xq, k)  # the full nq=10k batch: the schedule the bench runs
     assert idx.lastSearchInfo()["tensor_cores"] == 1
-    xb_host = xb.cpu().numpy()
-    ref.set_omp_threads(16)
-    rD, rI = ref.knn(xq[pick].cpu().numpy(), xb_host, k, 1)
+    rD, rI = ref_outputs_fullsize["flat_D"], ref_outputs_fullsize["flat_I"]
     gD, gI = D[pick].cpu().numpy(), I[pick].cpu().numpy()
     st = o.compare_lists(rD, rI, gD, gI, eps=1e-4, pct_max_diff1=0.01, pct_max_diffN=0.005)
     assert (rI == gI).mean() > 0.97, st
@@ -179,8 +228,7 @@ def test_flat_l2_10m_vs_reference(res, ref):
     idx.add(xbi)
     D, I = idx.search(xqi, k)
     assert idx.lastSearchInfo()["tensor_cores"] == 1
-    xb_host = xbi.cpu().numpy()
-    rD, rI = ref.knn(xqi[pick].cpu().numpy(), xb_host, k, 1)
+    rD, rI = ref_outputs_fullsize["flatint_D"], ref_outputs_fullsize["flatint_I"]
     gD, gI = D[pick].cpu().numpy(), I[pick].cpu().numpy()
     assert np.array_equal(rD, gD), "integer regime: distances must be bit-exact"
     for q in range(len(pick)):
@@ -191,7 +239,7 @@ def test_flat_l2_10m_vs_reference(res, ref):
         assert (gI[q, 1:][same] > gI[q, :-1][same]).all()
 
 
-def test_ivfflat_10m_vs_reference(res, ref):
+def test_ivfflat_10m_vs_reference(res, ref_outputs_fullsize):
     """configs[2]: GpuIndexIVFFlat N=10M nlist=4096 nprobe=64 k=100 vs faiss::IndexIVFFlat holding the same
     centroids and the same inverted lists (pulled with getListVectorData / getListIndices)."""
     import torch
@@ -199,35 +247,19 @@ def test_ivfflat_10m_vs_reference(res, ref):
     import faiss_b200 as fb
     from oracle import oracle_np as o
 
-    N, d, nlist, nprobe, nq, k = 10_000_000, 128, 4096, 64, 10_000, 100
-    idx = fb.GpuIndexIVFFlat(res, d, nlist, fb.METRIC_L2)
-    idx.setClustering(niter=4)
-    idx.train(_rows(torch, 1 << 19, d, 4321))
-    idx.reserveMemory(N + N // 8)
-    for c0 in range(0, N, 1_000_000):
-        idx.add(_rows(torch, 1_000_000, d, 1234 + c0 // 1_000_000))
+    N, d, nlist, nq, k = 10_000_000, 128, 4096, 10_000, 100
+    idx = ivfflat_10m_index(torch, fb, res)
     assert idx.ntotal == N
-    idx.nprobe = nprobe
+    assert sum(idx.getListLength(l) for l in range(nlist)) == N
     xq, pick = _sample_queries(torch, nq, d, 1235)
     D, I = idx.search(xq, k)
-    cpu = ref.IndexIVFFlat(d, nlist, 1)
-    cpu.set_centroids(idx.getCoarseCentroids())
-    cpu.set_is_trained(True)
-    tot = 0
-    for l in range(nlist):
-        ids = idx.getListIndices(l)
-        if ids.size:
-            cpu.add_entries(l, ids, idx.getListVectorData(l))
-            tot += ids.size
-    assert tot == N and cpu.ntotal == N
-    cpu.set_nprobe(nprobe)
-    rD, rI = cpu.search(xq[pick].cpu().numpy(), k)
+    rD, rI = ref_outputs_fullsize["ivfflat_D"], ref_outputs_fullsize["ivfflat_I"]
     gD, gI = D[pick].cpu().numpy(), I[pick].cpu().numpy()
     o.compare_lists(rD, rI, gD, gI, eps=1e-4, pct_max_diff1=0.02, pct_max_diffN=0.01)
     assert (rI == gI).mean() > 0.95
 
 
-def test_ivfpq_100m_vs_reference(res, ref):
+def test_ivfpq_100m_vs_reference(res, ref_outputs_fullsize):
     """configs[3]: GpuIndexIVFPQ N=100M nlist=4096 M=32 nprobe=32 k=100 vs faiss::IndexIVFPQ holding the same
     coarse centroids, PQ codebooks and list bytes (the clone direction of BASELINE.md section 3.4)."""
     import torch
@@ -235,32 +267,12 @@ def test_ivfpq_100m_vs_reference(res, ref):
     import faiss_b200 as fb
     from oracle import oracle_np as o
 
-    N, d, nlist, M, nprobe, nq, k = 100_000_000, 128, 4096, 32, 32, 10_000, 100
-    idx = fb.GpuIndexIVFPQ(res, d, nlist, M, 8, fb.METRIC_L2)
-    idx.setClustering(niter=4)
-    idx.setPQClustering(niter=4)
-    idx.train(_rows(torch, 1 << 19, d, 4321))
-    idx.reserveMemory(N + N // 8)
-    CH = 2_000_000
-    for c0 in range(0, N, CH):
-        idx.add(_rows(torch, CH, d, 1234 + c0 // CH, chunk=CH))
+    N, d, nq, k = 100_000_000, 128, 10_000, 100
+    idx = ivfpq_100m_index(torch, fb, res)
     assert idx.ntotal == N
-    idx.nprobe = nprobe
     xq, pick = _sample_queries(torch, nq, d, 1235)
     D, I = idx.search(xq, k)
-    cpu = ref.IndexIVFPQ(d, nlist, M, 8, 1)
-    cpu.set_centroids(idx.getCoarseCentroids())
-    cpu.set_pq_centroids(idx.getPQCentroids())
-    cpu.set_is_trained(True)
-    for l in range(nlist):
-        ids = idx.getListIndices(l)
-        if ids.size:
-            cpu.add_entries(l, ids, idx.getListVectorData(l))
-    assert cpu.ntotal == N
-    cpu.set_precomputed_table(0)
-    cpu.set_nprobe(nprobe)
-    ref.set_omp_threads(16)
-    rD, rI = cpu.search(xq[pick].cpu().numpy(), k)
+    rD, rI = ref_outputs_fullsize["ivfpq_D"], ref_outputs_fullsize["ivfpq_I"]
     gD, gI = D[pick].cpu().numpy(), I[pick].cpu().numpy()
     # PQ distances of 100M codes have many near-ties at rank ~100: ids may swap between adjacent ranks,
     # distances agree to fp32 summation order (the reference test's own tolerance is 0.035 / 0.1 / 0.06)

@@ -1,6 +1,6 @@
 """Pins the numpy oracle (oracle/oracle_np.py) against the reference: golden fixtures generated
-from the unmodified reference CPU library (tests/golden/make_golden.py) and, where oracle/_ref is
-present, the library itself.  No GPU needed."""
+from the unmodified reference CPU library (tests/golden/make_golden.py and
+tests/golden/make_reference_outputs.py).  No GPU needed."""
 import numpy as np
 import pytest
 
@@ -145,59 +145,79 @@ def test_kmeans_spherical_ip_oracle_vs_golden(golden):
     assert np.allclose(np.linalg.norm(cent, axis=1), 1.0, atol=1e-5)
 
 
-# ------------------------------------------------------------------ live checks against oracle/_ref
-def test_flat_vs_reference_live(ref):
+# ------------------------------------------------------------------ checks against the reference library's own answers
+# (stored by tests/golden/make_reference_outputs.py from oracle/_ref; the inputs are regenerated here from the same seeds)
+FLAT_LIVE_CASES = [(2000, 16, 30, 5, 1), (1500, 40, 11, 120, 0), (50, 8, 4, 60, 1)]
+
+
+def flat_live_inputs():
+    """(xb, xq, k, metric) per FLAT_LIVE_CASES entry"""
     rs = np.random.RandomState(0)
-    for (N, d, nq, k, metric) in [(2000, 16, 30, 5, 1), (1500, 40, 11, 120, 0), (50, 8, 4, 60, 1)]:
+    for (N, d, nq, k, metric) in FLAT_LIVE_CASES:
         xb = rs.rand(N, d).astype(np.float32)
         xq = rs.rand(nq, d).astype(np.float32)
-        idx = ref.IndexFlat(d, metric)
-        idx.add(xb)
-        rD, rI = idx.search(xq, k)
+        yield xb, xq, k, metric
+
+
+def precomputed_onoff_inputs():
+    """xb, xq of test_precomputed_table_on_off_same_ids: IndexIVFPQ(d=16, nlist=8, M=4), niter 4, nprobe 3, k 10"""
+    rs = np.random.RandomState(1)
+    xb = rs.rand(4000, 16).astype(np.float32)
+    xq = rs.rand(20, 16).astype(np.float32)
+    return xb, xq
+
+
+def precomputed_form_inputs():
+    """xb, xq of test_oracle_precomputed_form_vs_reference: IndexIVFPQ(d=32, nlist=16, M=8), niter 4, nprobe 4, k 10"""
+    rs = np.random.RandomState(7)
+    xb = rs.rand(6000, 32).astype(np.float32)
+    xq = rs.rand(30, 32).astype(np.float32)
+    return xb, xq
+
+
+def stored_lists(outputs, prefix, xb):
+    """per-list codes and ids of a reference IndexIVFPQ stored by make_reference_outputs.py: the oracle's encoding of each
+    vector's residual to its stored list, with the stored codes where the reference's differ (fp near-ties)"""
+    cent, pq, a = outputs[prefix + "_centroids"], outputs[prefix + "_pq"], outputs[prefix + "_list"].astype(np.int64)
+    rows = outputs[prefix + "_patch_rows"]
+    assert rows.size <= xb.shape[0] * 0.002  # the restatement of compute_code agrees but for near-ties
+    codes = o.pq_encode(xb - cent[a], pq)
+    codes[rows] = outputs[prefix + "_patch_codes"]
+    li = [np.flatnonzero(a == l) for l in range(cent.shape[0])]
+    return [codes[i].reshape(-1) for i in li], li
+
+
+def test_flat_vs_reference_live(ref_outputs):
+    for i, (xb, xq, k, metric) in enumerate(flat_live_inputs()):
+        rD, rI = ref_outputs["flat_%d_D" % i], ref_outputs["flat_%d_I" % i]
         D, I = o.knn_flat(xq, xb, k, metric)
         o.compare_lists(rD, rI, D, I, eps=1e-4, pct_max_diff1=0.02, pct_max_diffN=0.01)
 
 
-def test_precomputed_table_on_off_same_ids(ref):
+def test_precomputed_table_on_off_same_ids(ref_outputs):
     """tests/test_index_accuracy.py:506-508: precomputed table on/off gives identical ids; the
     oracle's residual form is therefore a faithful restatement of either mode."""
-    rs = np.random.RandomState(1)
-    xb = rs.rand(4000, 16).astype(np.float32)
-    xq = rs.rand(20, 16).astype(np.float32)
-    ivf = ref.IndexIVFPQ(16, 8, 4, 8, 1)
-    ivf.set_cp(niter=4)
-    ivf.set_pq_cp(niter=4)
-    ivf.train(xb)
-    ivf.add(xb)
-    ivf.set_nprobe(3)
-    ivf.set_precomputed_table(1)
-    D1, I1 = ivf.search(xq, 10)
-    ivf.set_precomputed_table(0)
-    D0, I0 = ivf.search(xq, 10)
+    xb, xq = precomputed_onoff_inputs()
+    D1, I1 = ref_outputs["onoff_D1"], ref_outputs["onoff_I1"]
+    D0, I0 = ref_outputs["onoff_D0"], ref_outputs["onoff_I0"]
     assert (I0 == I1).mean() > 0.98
     assert np.allclose(D0, D1, rtol=1e-4, atol=1e-5)
+    # the stored index is the one the reference trained on these inputs: the oracle reproduces its lists and answers
+    cent, pq = ref_outputs["onoff_centroids"], ref_outputs["onoff_pq"]
+    lc, li = stored_lists(ref_outputs, "onoff", xb)
+    D, I = o.ivfpq_search(xq, 10, 3, cent, pq, lc, li, 1, precomputed=False)
+    o.compare_lists(D0, I0, D, I, eps=1e-4, pct_max_diff1=0.02, pct_max_diffN=0.01)
 
 
-def test_oracle_precomputed_form_vs_reference(ref):
+def test_oracle_precomputed_form_vs_reference(ref_outputs):
     """the numpy restatement of the precomputed-table decomposition (what the GPU scan evaluates when
     usePrecomputedTables is active) against the reference CPU index with use_precomputed_table = 1, and
     against the residual form: same ids up to near-ties, distances within 1e-4 relative"""
-    rs = np.random.RandomState(7)
-    d, nlist, M, k, nprobe = 32, 16, 8, 10, 4
-    xb = rs.rand(6000, d).astype(np.float32)
-    xq = rs.rand(30, d).astype(np.float32)
-    ivf = ref.IndexIVFPQ(d, nlist, M, 8, 1)
-    ivf.set_cp(niter=4)
-    ivf.set_pq_cp(niter=4)
-    ivf.train(xb)
-    ivf.add(xb)
-    ivf.set_nprobe(nprobe)
-    ivf.set_precomputed_table(1)
-    rD, rI = ivf.search(xq, k)
-    cent = ivf.centroids()
-    pq = ivf.pq_centroids()
-    lists = [ivf.get_list(l) for l in range(nlist)]
-    lc, li = [c for c, _ in lists], [i for _, i in lists]
+    xb, xq = precomputed_form_inputs()
+    k, nprobe = 10, 4
+    rD, rI = ref_outputs["pcform_D"], ref_outputs["pcform_I"]
+    cent, pq = ref_outputs["pcform_centroids"], ref_outputs["pcform_pq"]
+    lc, li = stored_lists(ref_outputs, "pcform", xb)
     D1, I1 = o.ivfpq_search(xq, k, nprobe, cent, pq, lc, li, 1, precomputed=True)
     D0, I0 = o.ivfpq_search(xq, k, nprobe, cent, pq, lc, li, 1, precomputed=False)
     o.compare_lists(rD, rI, D1, I1, eps=1e-4, pct_max_diff1=0.02, pct_max_diffN=0.01)
